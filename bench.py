@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16x3|bf16x3|fp16|bf16]
                     [--config cfg2|cfg3|cfg5] [--scaling weak|strong] [--gather maps|labels|none]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over one frame of rays (default: config 2 of BASELINE.json, 376 x 1408 rays,
 64 samples/ray, 8 x 256 MLP, rgb + sigma, 64 bounding primitives) through the public API - Renderer.render, i.e.
@@ -18,6 +19,11 @@ e2e    : the same through Renderer.render from pinned HOST rays, H2D + D2H insid
 roofline: dominant kernel (fused MLP) algorithmic FLOP/s vs the measured dense bf16 tensor peak
 cpu_baseline / --impl reference: the CPU oracle (port of the spec; the reference source is not in the
          mount) timed on the box's host cores on a bounded strip of the same frame.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes every tensor the last timed step returned (Renderer.render's
+dict, plus the gathered tiles as gathered_<name> when there is a gather) as DIR/<name>.npy, float32 (float64 stays
+float64; integer and mask outputs are converted exactly).  The inputs are seeded, so two builds run with the same
+arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -216,8 +222,10 @@ def run_reference(args, cfg, rank, world):
         orc.run(rows)
     secs = []
     for _ in range(args.steps):
-        _, dt, _, _ = orc.run(rows)
+        _, dt, _, out = orc.run(rows)
         secs.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     rays = rows * cfg.W_img
     value = rays * len(secs) / sum(secs)
     sample = (f"{rows}-row strip ({rays} rays) of the {cfg.H}x{cfg.W_img} frame per step; median step "
@@ -255,6 +263,30 @@ def parity_on_strip(ref_out, gpu_out, far: float) -> dict:
     return rep
 
 
+DUMP_BUDGET = 60 << 20      # bytes of array data under --dump-outputs; the .npy headers add ~128 bytes per file
+
+
+def dump_outputs(dirname: str, arrays: dict) -> None:
+    """Write each tensor of `arrays` as <dirname>/<name>.npy: float64 stays float64, everything else becomes float32
+    (exact for the integer ids, labels and masks).  When the whole set exceeds DUMP_BUDGET, every tensor keeps the same
+    fixed, seeded sample of its rows (first dimension, ascending), so a file holds the same rays in every run."""
+    import numpy as np
+    arrays = {k: v.detach() for k, v in arrays.items() if torch.is_tensor(v)}
+    total = sum(v.numel() * (8 if v.dtype == torch.float64 else 4) for v in arrays.values())
+    keep = min(1.0, DUMP_BUDGET / total) if total else 1.0
+    rows = {}
+    d = Path(dirname)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in sorted(arrays.items()):
+        if keep < 1.0 and t.dim() > 0:
+            n = t.shape[0]
+            if n not in rows:
+                rows[n] = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:int(n * keep)].sort().values
+            t = t[rows[n].to(t.device)]
+        t = t.cpu().to(torch.float64 if t.dtype == torch.float64 else torch.float32)
+        np.save(d / f"{name}.npy", t.numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -270,6 +302,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fast-mode", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg3 block under 'extra'")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (at most 64 MB: a fixed, seeded sample "
+                         "of the rays when the frame's outputs are larger)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
@@ -357,6 +392,8 @@ def main():
     total_ms = float(total_ms.item())
     value = R_total * args.steps / (total_ms / 1e3)
     assert torch.isfinite(out["rgb_map"]).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {**out, **{f"gathered_{k}": v for k, v in (gathered or {}).items()}})
     gather_bytes = None
     if gathered is not None:
         gather_bytes = int(gathered["bytes_per_rank"]) if args.gather == "labels" else 20 * math.ceil(R_gather / world)

@@ -2,7 +2,7 @@
     python tests/golden/make_golden.py
 The reference has no golden vectors (its source is not in the mount), so these fixtures pin the ORACLE
 against drift and give the GPU tests a committed target that does not depend on importing anything at
-run time.  Inputs are seeded; everything is fp32/int32 and small (< 1 MB)."""
+run time.  Inputs are seeded; everything is fp32/int32/int64 and the file is small (< 1 MB, see save_deflated)."""
 import sys
 from pathlib import Path
 
@@ -57,7 +57,24 @@ def build():
     return out
 
 
+def save_deflated(obj, dst: Path) -> None:
+    """torch.save stores its zip members uncompressed (1.09 MB for these fixtures).  Deflating the members that
+    deflate to under half their size (integer ids, indices, the pickle) keeps the file under 1 MB; the random
+    fp32 members stay stored.  torch.load reads both kinds of member."""
+    import io
+    import zipfile
+    import zlib
+    buf = io.BytesIO()
+    torch.save(obj, buf)
+    with zipfile.ZipFile(buf) as src, zipfile.ZipFile(dst, "w") as out:
+        for member in src.infolist():
+            data = src.read(member.filename)
+            deflate = len(zlib.compress(data, 9)) < len(data) // 2
+            out.writestr(member.filename, data, compress_type=zipfile.ZIP_DEFLATED if deflate else zipfile.ZIP_STORED,
+                         compresslevel=9)
+
+
 if __name__ == "__main__":
     dst = Path(__file__).with_name("render_golden.pt")
-    torch.save(build(), dst)
+    save_deflated(build(), dst)
     print(dst, dst.stat().st_size, "bytes")

@@ -44,3 +44,18 @@ def test_reference_arm_under_torchrun_only_rank0_reports():
               "--master-addr", "127.0.0.1", "--master-port", str(_free_port()), "bench.py", "--impl", "reference",
               "--gpus", "2", "--steps", "1", "--warmup", "1", "--ref-rows", "1"])
     _check(d, 2)
+
+
+def test_reference_arm_dumps_the_same_outputs_every_run(tmp_path):
+    """--dump-outputs DIR: the last step's outputs as float32 / float64 .npy files, identical from run to run."""
+    import numpy as np
+    runs = []
+    for i in range(2):
+        d = tmp_path / str(i)
+        _check(_run([sys.executable, "bench.py", "--impl", "reference", "--steps", "1", "--warmup", "1", "--ref-rows", "1",
+                     "--dump-outputs", str(d)]), 1)
+        runs.append({p.name: np.load(p) for p in sorted(d.glob("*.npy"))})
+    assert {"rgb_map.npy", "depth_map.npy", "acc_map.npy", "weights.npy"} <= set(runs[0]) and runs[0].keys() == runs[1].keys()
+    for name, a in runs[0].items():
+        assert a.dtype in (np.float32, np.float64), name
+        assert np.array_equal(a, runs[1][name], equal_nan=True), name
