@@ -405,6 +405,60 @@ int pnr_comm_init(pnr_comm** out, const uint8_t* id, int32_t rank, int32_t world
 int pnr_comm_destroy(pnr_comm* comm);
 int pnr_allgather_outputs(pnr_comm* comm, const void* send, void* recv, size_t bytes_per_rank, void* stream);
 
+/* Evaluation of rendered frames (the reference's `run.py --type evaluate` / lib/evaluators): every frame passed to
+ * pnr_eval_frame is ACCUMULATED into a caller-owned device statistics buffer; nothing is copied to the host per frame.
+ * Every input pair is optional (both NULL skips that metric family); all arrays are device pointers, R rays per frame.
+ *   semantic   sem_pred [R] i16 (pnr_label_tiles / pnr_panoptic_fuse labels), sem_gt [R] i32: confusion matrix, row =
+ *              GT, column = prediction; GT outside [0, C) and predictions outside [0, C) (-1) are ignored.  C <= 64.
+ *   panoptic   pan_pred / pan_gt [R] i32, ids category * label_divisor + instance (pnr_panoptic_fuse's convention with
+ *              label_divisor 1000), is_thing [C] u8.  A pixel is void when its id is negative or its category is
+ *              outside [0, C).  A stuff category (is_thing 0) has one segment: the instance part is dropped.  GT pixels of
+ *              a thing category with instance 0 are that category's crowd region.  A predicted segment p and a non-crowd
+ *              GT segment g of the same category match iff IoU = |p∩g| / (|p| + |g| - |p∩g| - |p ∩ GT-void|) > 0.5
+ *              (strict; the match is then unique).  TP = matches, FN = unmatched non-crowd GT segments, FP = unmatched
+ *              predicted segments except those with (|p ∩ GT-void| + |p ∩ crowd(category)|) / |p| > 0.5.  Per category:
+ *              TP / FP / FN and the sum of the TPs' IoUs.  At most PNR_EVAL_MAX_SEGMENTS distinct segments per side and
+ *              frame: a frame with more adds no PQ terms and increments the overflow word instead.
+ *   image      rgb_pred / rgb_gt [R,3] f32: PSNR = -10 log10(mean squared error over the R*3 values), per frame.  With
+ *              H * W == R (rays row-major; H = W = 0 skips it): SSIM (Wang et al. 2004) with an 11x11 Gaussian window
+ *              (sigma 1.5, separable, normalised), valid region only, c1 = 0.01^2, c2 = 0.03^2, data range 1, variances
+ *              clamped at 0, mean over the valid pixels and the 3 channels, window moments in fp64.
+ *   depth      depth_pred / depth_gt [R] f32: pixels with 0 < gt <= max_depth count, the prediction is clamped to
+ *              [min_depth, max_depth] (min_depth > 0); sums in fp64 of |d|/gt, d^2/gt, d^2, (log p - log gt)^2 and the
+ *              counts of valid pixels and of max(p/gt, gt/p) < 1.25, 1.25^2, 1.25^3.
+ * Statistics layout (pnr_eval_stats_bytes(C) bytes, 8-byte words; zero it once, then pass frames): the words
+ * PNR_EVAL_* below (i64 counts, f64 sums), then from word PNR_EVAL_HEADER_WORDS: conf i64 [C*C], tp i64 [C], fp i64 [C],
+ * fn i64 [C], iou_sum f64 [C].  Integer statistics are added with integer atomics, floating-point sums in a fixed order
+ * (per-block partials summed by one thread; frames added in call order): the buffer is bit-identical from run to run.
+ * workspace: pnr_eval_workspace_bytes(R, C, label_divisor) bytes (256-byte aligned; label_divisor <= 0 when no panoptic
+ * inputs are passed), reused by every frame on the same stream.  Arguments are checked before any CUDA call. */
+#define PNR_EVAL_MAX_CLASSES 64
+#define PNR_EVAL_MAX_SEGMENTS 1024
+#define PNR_EVAL_MAX_KEYS (1 << 24)   /* C * label_divisor */
+#define PNR_EVAL_HEADER_WORDS 16
+enum { PNR_EVAL_OVERFLOW = 0,      /* i64: frames whose segments exceeded PNR_EVAL_MAX_SEGMENTS (no PQ terms added) */
+       PNR_EVAL_PQ_FRAMES = 1,     /* i64: frames that added PQ terms                                          */
+       PNR_EVAL_PSNR_FRAMES = 2,   /* i64 */
+       PNR_EVAL_SSIM_FRAMES = 3,   /* i64 */
+       PNR_EVAL_DEPTH_VALID = 4,   /* i64, then DELTA1..3 (i64) in words 5..7                                    */
+       PNR_EVAL_DEPTH_DELTA1 = 5, PNR_EVAL_DEPTH_DELTA2 = 6, PNR_EVAL_DEPTH_DELTA3 = 7,
+       PNR_EVAL_PSNR_SUM = 8,      /* f64: sum of the per-frame PSNRs (dB)                                     */
+       PNR_EVAL_SSIM_SUM = 9,      /* f64: sum of the per-frame SSIMs                                           */
+       PNR_EVAL_ABS_REL_SUM = 10, PNR_EVAL_SQ_REL_SUM = 11, PNR_EVAL_SQ_ERR_SUM = 12, PNR_EVAL_SQ_LOG_SUM = 13
+       /* words 14, 15: reserved, zero */ };
+typedef struct pnr_eval_args {
+  int64_t R; int32_t C; int32_t H, W;                  /* H*W == R enables SSIM, else 0, 0                          */
+  const int16_t* sem_pred; const int32_t* sem_gt;
+  const int32_t* pan_pred; const int32_t* pan_gt; const uint8_t* is_thing; int32_t label_divisor;
+  const float* rgb_pred; const float* rgb_gt;
+  const float* depth_pred; const float* depth_gt; float min_depth, max_depth;
+  void* stats;                                         /* pnr_eval_stats_bytes(C), zeroed once, accumulated         */
+  void* workspace; size_t workspace_bytes;             /* pnr_eval_workspace_bytes(R, C, label_divisor)             */
+} pnr_eval_args;
+size_t pnr_eval_stats_bytes(int32_t C);
+size_t pnr_eval_workspace_bytes(int64_t R, int32_t C, int32_t label_divisor);
+int pnr_eval_frame(const pnr_eval_args* args, void* stream);
+
 /* Number of kernels this library has launched on this thread since the last reset (bench evidence). */
 int64_t pnr_launch_count(int32_t reset);
 

@@ -4,12 +4,17 @@ batchify_rays, raw2outputs, sample_pdf).  All compute is hand-written CUDA in li
 include/pnr.h); there is no CPU or PyTorch fallback."""
 from .config import make_cfg, PRESETS  # noqa: F401
 
-__all__ = ["make_cfg", "PRESETS", "make_network", "make_renderer"]
+__all__ = ["make_cfg", "PRESETS", "make_network", "make_renderer", "make_evaluator"]
 
 
 def make_network(cfg):
     from .lib.networks import make_network as _mk
     return _mk(cfg)
+
+
+def make_evaluator(cfg, device=None):
+    from .lib.evaluators import make_evaluator as _mk
+    return _mk(cfg, device)
 
 
 def make_renderer(cfg, network, network_fine=None):

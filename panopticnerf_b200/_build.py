@@ -14,7 +14,8 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libpnr.so"
-SOURCES = ["pnr_api.cu", "ray_kernels.cu", "stream_kernels.cu", "mlp_tc05.cu", "render.cu", "comm.cu", "panoptic_kernels.cu", "wgrad_tc05.cu", "linear_tc05.cu"]
+SOURCES = ["pnr_api.cu", "ray_kernels.cu", "stream_kernels.cu", "mlp_tc05.cu", "render.cu", "comm.cu", "panoptic_kernels.cu", "wgrad_tc05.cu", "linear_tc05.cu",
+           "eval_kernels.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"] + os.environ.get("PNR_NVCC_FLAGS", "").split()   # e.g. -DPNR_TIMELINE
 

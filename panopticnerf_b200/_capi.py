@@ -66,6 +66,16 @@ class PnrRenderArgs(C.Structure):
                 ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
 
 
+class PnrEvalArgs(C.Structure):
+    """pnr_eval_args of include/pnr.h (same field order)."""
+    _fields_ = [("R", C.c_int64), ("C", C.c_int32), ("H", C.c_int32), ("W", C.c_int32)] + \
+               [(k, C.c_void_p) for k in ("sem_pred", "sem_gt", "pan_pred", "pan_gt", "is_thing")] + \
+               [("label_divisor", C.c_int32)] + \
+               [(k, C.c_void_p) for k in ("rgb_pred", "rgb_gt", "depth_pred", "depth_gt")] + \
+               [("min_depth", C.c_float), ("max_depth", C.c_float), ("stats", C.c_void_p), ("workspace", C.c_void_p),
+                ("workspace_bytes", C.c_size_t)]
+
+
 SAMPLE_MODE = {"uniform": 0, "intervals": 1}
 COMM_ID_BYTES = 128
 
@@ -118,6 +128,9 @@ SIGNATURES = {
     "pnr_comm_init": (C.c_int, [C.POINTER(_vp), C.POINTER(C.c_uint8), _i32, _i32, _i32]),
     "pnr_comm_destroy": (C.c_int, [_vp]),
     "pnr_allgather_outputs": (C.c_int, [_vp, _vp, _vp, C.c_size_t, _vp]),
+    "pnr_eval_stats_bytes": (C.c_size_t, [_i32]),
+    "pnr_eval_workspace_bytes": (C.c_size_t, [_i64, _i32, _i32]),
+    "pnr_eval_frame": (C.c_int, [C.POINTER(PnrEvalArgs), _vp]),
     "pnr_launch_count": (_i64, [_i32]),
 }
 
